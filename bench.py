@@ -7,6 +7,8 @@ configurations; N=1 is the local kernel with no ring).
   python bench.py --gpus N --steps K --warmup W            (N>1: launched under torchrun)
   python bench.py --impl reference ...                     CPU arm: the oracle port of the
                                                            reference's path on the host cores
+  python bench.py ... --dump-outputs DIR                   also write a sample of what the last
+                                                           timed step returned (dump_outputs)
 
 One "step" = one forward + one backward of burst_attn_func on synthetic
 N(0,1) bf16 inputs already resident in HBM (`value`), and the same through the
@@ -199,7 +201,7 @@ def run_reference_arm(args):
     threads = best_cpu_threads(shim)
     S, Hc = 4096, 8
     warm = max(0, min(args.warmup, 1))
-    steps = max(1, min(args.steps, 5))
+    steps = args.steps
     t = 0.0
     if shim is not None:
         for _ in range(warm):
@@ -331,6 +333,24 @@ def ncu_traffic(kernel, Sq, Sk, Hh, causal):
     return (ent["dram_bytes"], ent.get("source")) if ent else (None, None)
 
 
+DUMP_ROWS = 512  # token positions over all ranks: 4 outputs x 512 x H x D x fp32 = 32 MiB at H=32, d=128
+
+
+def dump_outputs(dirname, outs, rank, world):
+    """Write (O, dQ, dK, dV) of one step, each [B, S_local, H, D], as <dirname>/{o,dq,dk,dv}.npy in float32, at
+    DUMP_ROWS // world token positions (all batch rows, heads and dims) drawn with a fixed seed.  The inputs are seeded
+    too, so the same arguments give the same positions of the same computation in every run: two builds can be
+    compared output for output.  With N > 1 ranks each writes a sample of its own shard as <name>_rank<r>.npy."""
+    import numpy as np
+    os.makedirs(dirname, exist_ok=True)
+    S_loc = outs[0].shape[1]
+    n = min(S_loc, max(1, DUMP_ROWS // world))
+    idx = torch.randperm(S_loc, generator=torch.Generator().manual_seed(0))[:n].sort().values.to(outs[0].device)
+    suffix = "" if world == 1 else f"_rank{rank}"
+    for name, t in zip(("o", "dq", "dk", "dv"), outs):
+        np.save(os.path.join(dirname, f"{name}{suffix}.npy"), t.detach().index_select(1, idx).float().cpu().numpy())
+
+
 # --------------------------------------------------------------------------- #
 def main():
     ap = argparse.ArgumentParser()
@@ -353,7 +373,16 @@ def main():
     ap.add_argument("--double-ring", type=int, default=0, metavar="L",
                     help="run over the hierarchical (double) ring with intra-node rings of L consecutive ranks "
                          "(reference benchmarks/benchmark.py --double_ring); default 0 = flat ring")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned (O, dQ, dK, dV) as DIR/<name>.npy, "
+                         "float32, at a fixed seeded sample of token positions (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
+    if args.dump_outputs and args.configs:
+        ap.error("--dump-outputs takes the one configuration of --seq / --causal, not --configs")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU path computed; --impl reference times a CPU sample instead")
 
     if args.impl == "reference":
         return run_reference_arm(args)
@@ -369,7 +398,7 @@ def main():
         dist.init_process_group("nccl", device_id=dev)
     assert world == args.gpus, f"--gpus {args.gpus} but WORLD_SIZE={world}"
     W = max(3, args.warmup)
-    K = max(1, args.steps)
+    K = args.steps
 
     from burst_attn import burst_attn_func
     from burst_attn import chunk_ops, native
@@ -420,6 +449,15 @@ def _bench_one(args, world, rank, local, dev, W, K, ops, burst_attn_func):
         dq, dk, dv = torch.autograd.grad(o, (qq, kk, vv), dod)
         return o, dq, dk, dv
 
+    # --dump-outputs keeps each step's results alive until the next step has returned; the warm-up does the same, so
+    # the extra memory is in the allocator's cache before the timed steps start
+    last = []
+
+    def bench_step():
+        res = step(q, k, v, do)
+        if args.dump_outputs:
+            last[:] = res
+
     def fwd_only(qd, kd, vd):
         with torch.no_grad():
             return burst_attn_func(qd, kd, vd, None, "cuda", args.causal, True, False, None, args.double_group)
@@ -444,7 +482,7 @@ def _bench_one(args, world, rank, local, dev, W, K, ops, burst_attn_func):
 
     # ---- warm-up (also builds the NCCL ring)
     for _ in range(W):
-        step(q, k, v, do)
+        bench_step()
     torch.cuda.synchronize()
 
     # ---- timed: fwd+bwd, inputs resident in HBM; per-kernel events on the launching stream
@@ -454,13 +492,16 @@ def _bench_one(args, world, rank, local, dev, W, K, ops, burst_attn_func):
     ops.enable_timing(True)
     launches0 = ops.launches
     t_wall0 = time.time()
-    ms_step = timed(lambda: step(q, k, v, do), K)
+    ms_step = timed(bench_step, K)
     t_wall1 = time.time()
     launches = ops.launches - launches0
     torch.cuda.synchronize()
     kms = ops.kernel_ms()
     ops.enable_timing(False)
     clocks = sampler.stop(t_wall0, t_wall1)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last, rank, world)
+        last.clear()
     ms_fwd = timed(lambda: fwd_only(q, k, v), max(1, min(K, 3)))
 
     causal_div = 2.0 if args.causal else 1.0

@@ -8,6 +8,14 @@ The reference imports `bmtrain` (absent here) at module scope
 reference source is modified or copied.
 
 Run:  python tests/golden/make_golden.py      (needs /root/reference)
+
+`ring` writes reference_cpu_ring.npz: the reference's whole CPU ring step (its own
+inter_normal_attn / inter_normal_attn_backward over a simulated ring, through
+baseline/ref_shim.py), which tests/test_oracle_golden.py pins the oracle's dense
+attention to.  It needs the reference installed in baseline/_ref, which build()
+makes where the reference's source is available.
+
+      python tests/golden/make_golden.py ring
 """
 import os
 import sys
@@ -18,6 +26,24 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 REF = "/root/reference"
+
+# inputs of the ring vectors: torch.manual_seed(RING_SEED), then q, k, v, dO = randn(RING_SHAPE) in that order,
+# layout [B, H, S, D]; of each 512 KB output RING_PER_ROW elements of every (b, h, s) row are stored, at columns
+# drawn with a fixed seed, so an error confined to a few rows (a chunk edge, say) is still seen
+RING_SEED, RING_SHAPE, RING_WORLDS, RING_PER_ROW = 0, (1, 4, 512, 64), (1, 4), 2
+
+
+def ring_inputs():
+    torch.manual_seed(RING_SEED)
+    return [torch.randn(*RING_SHAPE) for _ in range(4)]
+
+
+def ring_sample_index():
+    """Flat indices into a contiguous RING_SHAPE tensor, sorted."""
+    rows, D = int(np.prod(RING_SHAPE[:-1])), RING_SHAPE[-1]
+    g = torch.Generator().manual_seed(RING_SEED + 1)
+    cols = torch.rand(rows, D, generator=g).argsort(dim=1)[:, :RING_PER_ROW]
+    return (torch.arange(rows).unsqueeze(1) * D + cols).flatten().sort().values
 
 
 def _stub_bmtrain():
@@ -131,5 +157,23 @@ def main():
     print("wrote", os.path.join(HERE, "reference_vectors.npz"), sorted(out))
 
 
+def ring():
+    sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(HERE)), "baseline"))
+    import ref_shim
+    q, k, v, do = ring_inputs()
+    idx = ring_sample_index()
+    out = {"idx": idx.numpy().astype(np.int32)}
+    out.update({f"in_{n}": t.flatten()[idx].numpy() for n, t in zip(("q", "k", "v", "do"), (q, k, v, do))})
+    for W in RING_WORLDS:
+        o, dq, dk, dv, _, _ = ref_shim.cpu_ring_step(q, k, v, do, W, RING_SHAPE[-1] ** -0.5)
+        out.update({f"W{W}_{n}": t.flatten()[idx].numpy() for n, t in zip(("o", "dq", "dk", "dv"), (o, dq, dk, dv))})
+    path = os.path.join(HERE, "reference_cpu_ring.npz")
+    np.savez_compressed(path, **out)
+    print("wrote", path, sorted(out))
+
+
 if __name__ == "__main__":
-    main()
+    if sys.argv[1:] == ["ring"]:
+        ring()
+    else:
+        main()
